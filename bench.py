@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- keyframes/sec of the loop-closure front-end and pose-graph solve ms on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one batch of KF_PER_STEP = 10 four-view fisheye keyframes through the hot path (BASELINE.json config C3 per
@@ -12,6 +12,8 @@ GPU; the default 20 steps time 200 keyframes, SURVEY.md section 8d), each keyfra
 `value`  = keyframes/s with the u8 images already resident in HBM (whole job, all ranks).
 `e2e`    = the same through the host-buffer C-ABI call osb_frontend_process: pinned host images in, record + loop
            result back to the host, H2D/D2H inside the timed region.
+--dump-outputs DIR: the keyframe records and loop results of the last timed step of `value` (rank 0), one .npy per field.
+The images, weights and database are seeded, so the same arguments give the same inputs on every run.
 N > 1: one drone per GPU (weak scaling); every step ends with ONE NCCL all-gather of the fixed-size keyframe
 record (replaces LoopNet's LCM multicast) and each GPU ingests the N-1 foreign records into its remote database.
 The pose-graph solve (BASELINE config C5 graph: 2000 nodes / 12 000 factors) is single-GPU ("replicas only"): it is
@@ -72,9 +74,16 @@ def parse():
     p.add_argument("--no-trt-like", action="store_true")
     p.add_argument("--blocking-exchange", action="store_true",
                    help="N > 1: all-gather of round i between extract and ingest of round i (the r01 pipeline), for A/B")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the keyframe records and loop results of the last timed step to DIR/<field>.npy")
     p.add_argument("--cpu-drone", type=int, default=-1, help=argparse.SUPPRESS)      # internal: one CPU drone of --impl reference
     p.add_argument("--cpu-threads", type=int, default=0, help=argparse.SUPPRESS)
-    return p.parse_args()
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes what the CUDA path computes: --impl ours only")
+    return a
 
 
 def peaks():
@@ -340,6 +349,10 @@ def run_ours(args):
     dev_dn = [t.cuda() for t in pin_dn]
     rec_dev = torch.zeros(lib.RECORD_BYTES, dtype=torch.uint8, device="cuda")
     res_dev = torch.zeros(lib.RESULT_BYTES, dtype=torch.uint8, device="cuda")
+    # the resident path writes keyframe k of a step to slot k, so after a step the slots hold everything it computed (N > 1:
+    # the asynchronous exchange reads a record one round later; a slot is rewritten only KF_PER_STEP rounds later)
+    rec_slots = [torch.zeros(lib.RECORD_BYTES, dtype=torch.uint8, device="cuda") for _ in range(KF_PER_STEP)]
+    res_slots = [torch.zeros(lib.RESULT_BYTES, dtype=torch.uint8, device="cuda") for _ in range(KF_PER_STEP)]
     gathered = torch.zeros(world * lib.RECORD_BYTES, dtype=torch.uint8, device="cuda") if world > 1 else None
     # N > 1: the exchange goes through the C ABI (osb_swarm_*: ncclAllGather on the library's own communicator); the
     # 128-byte communicator id travels over the torch.distributed group that also carries the timing reductions
@@ -388,15 +401,13 @@ def run_ours(args):
 
     def keyframe_resident(i):
         j = i % POOL
+        rec, res = rec_slots[i % KF_PER_STEP], res_slots[i % KF_PER_STEP]
+        fe.extract(dev_up[j].data_ptr(), dev_dn[j].data_ptr(), i, rec.data_ptr(), st, device_images=True)
         if world > 1:
-            rec = rec2[i & 1]
-            fe.extract(dev_up[j].data_ptr(), dev_dn[j].data_ptr(), i, rec.data_ptr(), st, device_images=True)
             swarm_round(i, rec)
-            fe.query(rec.data_ptr(), res_dev.data_ptr(), st)
         else:
-            fe.extract(dev_up[j].data_ptr(), dev_dn[j].data_ptr(), i, rec_dev.data_ptr(), st, device_images=True)
-            fe.ingest_own(rec_dev.data_ptr(), st)
-            fe.query(rec_dev.data_ptr(), res_dev.data_ptr(), st)
+            fe.ingest_own(rec.data_ptr(), st)
+        fe.query(rec.data_ptr(), res.data_ptr(), st)
 
     def keyframe_e2e(i):
         j = i % POOL
@@ -452,6 +463,7 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     sampler.start()
     ms_total, launches = timed(step_resident, args.steps, args.warmup, 0, sampler)
+    last_step = (torch.stack(rec_slots).cpu().numpy(), torch.stack(res_slots).cpu().numpy()) if args.dump_outputs else None
     # host cost of ENQUEUEING a keyframe with an empty launch queue (8 keyframes right after a synchronisation: no back-pressure)
     fe.finish(st); barrier()
     th = time.perf_counter()
@@ -924,12 +936,33 @@ def run_ours(args):
             line["trt_like_baseline"]["ours_e2e_over_trt_like"] = e2e_value / line["trt_like_baseline"]["value"]
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args)
+        if last_step:
+            dump_outputs(args.dump_outputs, *last_step)
         _emit(line)
     if world > 1:
         sw.wait(st); torch.cuda.synchronize()
         dist.barrier()
         sw.close()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, records, results):
+    """records [KF_PER_STEP, RECORD_BYTES] and results [KF_PER_STEP, RESULT_BYTES] (u8) -> out_dir/<field>.npy, one row per
+    keyframe of the step: every field of osb_keyframe_record and osb_loop_result, floats as float32, integers as float64
+    (exact).  List entries past their count (n_kpts per direction for the keypoint lists, n_matches / n_geo for the match
+    lists) carry no result and are written as 0."""
+    from omniswarm_b200 import lib
+    rec = np.frombuffer(records.tobytes(), np.dtype(lib.KeyframeRecord))
+    res = np.frombuffer(results.tobytes(), np.dtype(lib.LoopResult))
+    cols = {name: np.array(s[name]) for s in (rec, res) for name in s.dtype.names if name != "reserved"}
+    for count, names in (("n_kpts", ("local_desc", "kpts", "stereo_match", "landmarks_3d", "landmarks_flag")),
+                         ("n_matches", ("match_new", "match_old")), ("n_geo", ("geo_new", "geo_old"))):
+        past = np.arange(lib.MAX_KPTS)[None, None, :] >= cols[count][:, :, None]           # [keyframe, direction, entry]
+        for name in names:
+            cols[name][past] = 0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
 
 
 def _emit(line: dict):

@@ -7,9 +7,10 @@ it lies under /root/reference (nothing is copied into the repository), loads the
 and stores inputs and outputs as tests/golden/ref_superpoint.npz.
 
     python tests/golden/make_ref_superpoint.py          (needs /root/reference; the committed .npz travels without it)
+    python tests/golden/make_ref_superpoint.py --check  compare the committed fixture with the notebook instead of writing it
 
 tests/test_oracle_pins.py::test_network_oracle_matches_the_references_own_module compares oracle/frontend_ref.py with the
-fixture, and re-executes the notebook directly when the reference tree is present.
+fixture.
 """
 import json
 import os
@@ -57,7 +58,7 @@ def run_reference(img_u8, weights, scale="mul"):
     return semi[0].numpy().copy(), desc[0].numpy().copy()
 
 
-def main():
+def main(check=False):
     torch.set_num_threads(1)
     w = synth.superpoint_weights(0)
     out = {}
@@ -69,9 +70,15 @@ def main():
         out[f"desc_{seed}"] = desc
         if seed == 0:                                   # the notebook's own input scaling, for the record
             out["semi_div_0"], out["desc_div_0"] = run_reference(img, w, "div")
+    if check:
+        z = np.load(OUT)
+        assert sorted(z.files) == sorted(out) and all(np.array_equal(z[k], v) for k, v in out.items()), \
+            "tests/golden/ref_superpoint.npz differs from the notebook's outputs"
+        print("ref_superpoint.npz matches the notebook")
+        return
     np.savez_compressed(OUT, **out)
     print("wrote", OUT, {k: v.shape for k, v in out.items()})
 
 
 if __name__ == "__main__":
-    main()
+    main(check="--check" in sys.argv[1:])

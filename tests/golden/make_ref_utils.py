@@ -4,10 +4,12 @@ executed where they lie under /root/reference (their module imports the `transfo
 here, so only these function definitions are compiled); nothing is copied into the repository.
 
     python tests/golden/make_ref_utils.py        -> tests/golden/ref_utils.npz
+    python tests/golden/make_ref_utils.py --check   compare the committed fixture with the functions instead of writing it
 """
 import ast
 import math
 import os
+import sys
 
 import numpy as np
 
@@ -25,16 +27,23 @@ def reference_functions(names=("quat2eulers", "wrap_pi")):
     return [ns[n] for n in names]
 
 
-def main():
+def main(check=False):
     quat2eulers, wrap_pi = reference_functions()
     rng = np.random.default_rng(0)
     q = rng.standard_normal((200, 4))
     q /= np.linalg.norm(q, axis=1, keepdims=True)                     # wxyz
     ypr = np.array([quat2eulers(*row) for row in q])                  # the reference returns (yaw, pitch, roll)
     a = rng.uniform(-20, 20, 200)
-    np.savez(OUT, quat_wxyz=q, ypr=ypr, angle=a, wrapped=wrap_pi(a))
+    out = dict(quat_wxyz=q, ypr=ypr, angle=a, wrapped=wrap_pi(a))
+    if check:
+        z = np.load(OUT)
+        assert sorted(z.files) == sorted(out) and all(np.array_equal(z[k], v) for k, v in out.items()), \
+            "tests/golden/ref_utils.npz differs from the reference's functions"
+        print("ref_utils.npz matches the reference's functions")
+        return
+    np.savez(OUT, **out)
     print("wrote", OUT)
 
 
 if __name__ == "__main__":
-    main()
+    main(check="--check" in sys.argv[1:])

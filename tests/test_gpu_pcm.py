@@ -1,13 +1,18 @@
-"""GPU parity of the PCM outlier rejection (osb_pcm: pairwise consistency + FMC::maxCliqueHeu) against oracle/pcm_ref.py."""
+"""GPU parity of the PCM outlier rejection (osb_pcm: pairwise consistency + FMC::maxCliqueHeu) against oracle/pcm_ref.py, and
+against the clique the REFERENCE's own maxCliqueHeu finds on the oracle's consistency graph (tests/golden/ref_fmc.npz, written
+by tests/golden/make_ref_fmc.py from the library oracle/ref_build compiles from its sources)."""
+import os
+
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from omniswarm_b200 import synth, host
 from oracle import pcm_ref as pr
-from oracle import fmc_ref
 
 pytestmark = pytest.mark.gpu
 THRES, POS, ANG = 15.0, 1e-4, 1e-5
+REF_FMC = np.load(os.path.join(GOLDEN, "ref_fmc.npz"))
 
 
 @pytest.mark.parametrize("n,out,seed", [(60, 0.3, 0), (150, 0.5, 1), (33, 0.0, 2), (1, 0.0, 3)])
@@ -23,8 +28,7 @@ def test_pcm_matches_oracle(gpu, n, out, seed):
     assert np.array_equal(adj, radj)                                  # consistency graph bit-exact
     rclique, rsize = pr.max_clique_heu(radj)
     assert clique.tolist() == rclique                                 # same vertices in maxCliqueHeu's order
-    if fmc_ref.available():                                           # ... and in the order of the REFERENCE's own library
-        assert clique.tolist() == fmc_ref.max_clique_heu(radj)[0]     # (oracle/_ref/libfmc_ref.so, built from its sources)
+    assert clique.tolist() == REF_FMC[f"pcm_{n}_{seed}"].tolist()     # ... and in the order of the REFERENCE's own library
     if n > 30:
         assert all(edges[i]["inlier"] for i in clique) and len(clique) >= 0.4 * sum(e["inlier"] for e in edges)
 
@@ -45,8 +49,7 @@ def test_pcm_large_graph_bitmatrix_in_global_memory(gpu):
         assert adj[i, j] == (s < THRES)
     rclique, _ = pr.max_clique_heu(adj)
     assert clique.tolist() == rclique
-    if fmc_ref.available():
-        assert clique.tolist() == fmc_ref.max_clique_heu(adj)[0]
+    assert clique.tolist() == REF_FMC[f"pcm_{n}_5"].tolist()          # the reference's library on the oracle's graph
     assert all(edges[i]["inlier"] for i in clique) and len(clique) > 100
 
 

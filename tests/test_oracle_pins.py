@@ -383,8 +383,8 @@ def test_network_oracle_matches_the_references_own_module():
     """The SuperPoint stage of the oracle against the REFERENCE ITSELF: tests/golden/ref_superpoint.npz holds the outputs of the
     `SuperPointNet` class of swarm_loop/superpoint.ipynb (the module the reference exports its TensorRT engine from),
     executed in place by tests/golden/make_ref_superpoint.py with the seeded weights.  oracle/frontend_ref.py must
-    reproduce them (same torch kernels underneath: a few ulp); with the reference tree present the notebook is executed
-    again, so the fixture cannot drift from it."""
+    reproduce them (same torch kernels underneath: a few ulp).  `make_ref_superpoint.py --check` executes the notebook again
+    and compares its outputs with the fixture."""
     import os
     from oracle import frontend_ref as fr
     from omniswarm_b200 import synth
@@ -405,21 +405,12 @@ def test_network_oracle_matches_the_references_own_module():
     # oracle restates): one ulp on some pixels, a few 1e-6 on the heat map
     semi0, _ = fr.superpoint_net(z["img_0"], w, num_threads=1)
     assert 0 < np.abs(semi0 - z["semi_div_0"]).max() < 1e-5
-    if os.path.exists("/root/reference/swarm_loop/superpoint.ipynb"):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("make_ref_superpoint", os.path.join(here, "golden", "make_ref_superpoint.py"))
-        m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
-        import torch
-        torch.set_num_threads(1)
-        s = seeds[0]
-        semi_r, desc_r = m.run_reference(z[f"img_{s}"], w)
-        assert np.array_equal(semi_r, z[f"semi_{s}"]) and np.array_equal(desc_r, z[f"desc_{s}"])
 
 
 def test_euler_convention_matches_the_references_python_helpers():
     """`quat2eulers` and the angle wrap that the PnP / PCM oracles define (their C++ originals live in swarm_msgs, which is not in
     the tree) against the reference's own Python statement of them, swarm_localization/scripts/utils.py, executed in place by
-    tests/golden/make_ref_utils.py."""
+    tests/golden/make_ref_utils.py (`--check` compares them with the fixture again)."""
     import os
     from oracle import pnp_ref as pr
     from oracle import solver_ref as sr
@@ -430,38 +421,31 @@ def test_euler_convention_matches_the_references_python_helpers():
         assert np.allclose(rpy[::-1], ypr, atol=1e-12)                # the reference returns (yaw, pitch, roll)
     for a, w in zip(z["angle"], z["wrapped"]):
         assert abs(pr.wrap(a) - w) < 1e-12 and abs(sr.normalize_angle(a) - w) < 1e-12
-    if os.path.exists("/root/reference/swarm_localization/scripts/utils.py"):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("make_ref_utils", os.path.join(here, "golden", "make_ref_utils.py"))
-        m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
-        q2e, _ = m.reference_functions()
-        assert np.allclose(q2e(*z["quat_wxyz"][0]), z["ypr"][0], atol=0)
+
+
+def ref_fmc_graphs():
+    """the graphs of tests/golden/ref_fmc.npz with the clique and size the reference's own maxCliqueHeu returned on each"""
+    z = np.load(os.path.join(GOLDEN, "ref_fmc.npz"))
+    adj_end, clq_end = np.cumsum(z["pin_adj_bytes"]), np.cumsum(z["pin_clique_len"])
+    for g, n in enumerate(z["pin_n"]):
+        iu = np.triu_indices(n, 1)
+        a = np.zeros((n, n), np.uint8)
+        a[iu] = np.unpackbits(z["pin_adj"][adj_end[g] - z["pin_adj_bytes"][g]:adj_end[g]])[:len(iu[0])]
+        yield a | a.T, z["pin_clique"][clq_end[g] - z["pin_clique_len"][g]:clq_end[g]].tolist(), int(z["pin_size"][g])
 
 
 def test_max_clique_restatement_equals_the_references_own_library():
     """FMC::maxCliqueHeu is plain C++ inside the reference tree (third_party/fast_max-clique_finder), so it is COMPILED from its
-    sources in place (oracle/ref_build/Makefile -> oracle/_ref/libfmc_ref.so, nothing copied) and the restatement in
-    oracle/pcm_ref.py -- what the CUDA clique kernel is compared with -- must return the same clique, vertex by vertex in the
-    same order, on random graphs of every density and on the degenerate ones."""
+    sources in place (oracle/ref_build/Makefile -> oracle/_ref/libfmc_ref.so, nothing copied); tests/golden/ref_fmc.npz holds
+    what it returns on 423 graphs of every density, PCM-shaped and degenerate ones (tests/golden/make_ref_fmc.py).  The
+    restatement in oracle/pcm_ref.py -- what the CUDA clique kernel is compared with -- must return the same clique, vertex by
+    vertex in the same order; where the library has been built, it is asked again, so the fixture cannot drift from it."""
     from oracle import fmc_ref, pcm_ref
-    if not fmc_ref.build():
-        pytest.skip("oracle/_ref/libfmc_ref.so is not built and the reference tree is not here to build it from")
-    rng = np.random.default_rng(1)
-    graphs = [np.zeros((1, 1), np.uint8), np.zeros((7, 7), np.uint8), (1 - np.eye(9, dtype=np.uint8))]
-    for _ in range(400):
-        n = int(rng.integers(2, 60))
-        a = np.triu(rng.uniform(size=(n, n)) < rng.uniform(0.02, 0.95), 1)
-        graphs.append((a | a.T).astype(np.uint8))
-    # PCM-shaped graphs: a big consistent block plus scattered false links
-    for _ in range(20):
-        n = int(rng.integers(30, 120)); k = int(0.5 * n)
-        a = np.zeros((n, n), bool)
-        idx = rng.choice(n, k, replace=False)
-        a[np.ix_(idx, idx)] = True
-        a |= np.triu(rng.uniform(size=(n, n)) < 0.05, 1); a = np.triu(a, 1); a = a | a.T
-        graphs.append(a.astype(np.uint8))
-    for a in graphs:
-        ref_clique, ref_size = fmc_ref.max_clique_heu(a)
+    graphs = list(ref_fmc_graphs())
+    assert len(graphs) == 423
+    for a, ref_clique, ref_size in graphs:
         clique, size = pcm_ref.max_clique_heu(a)
         assert clique == ref_clique and size == ref_size
         assert all(a[u, v] for i, u in enumerate(clique) for v in clique[i + 1:])      # and it is a clique
+        if fmc_ref.available():
+            assert fmc_ref.max_clique_heu(a) == (ref_clique, ref_size)
